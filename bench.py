@@ -61,6 +61,8 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle comparison of the legs' output (outside the timed regions)")
     ap.add_argument("--flags", type=int, default=0, help="extra DNZ_FLAG_* bits for the operator (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the rows the last of them emitted to DIR/<column>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -287,6 +289,87 @@ def oracle_sample(wl, batches, sample_rows):
     return tab, cut, dt
 
 
+class StepCapture(list):
+    """The device results a step emits, copied on the operator's stream as each one is handed out (a result is valid only until
+    the next call on the operator), into a buffer of `reserve` bytes allocated up front (beyond it, into fresh allocations).
+    Capturing a timed step this way adds device-to-device copies to it but no host wait and, while the buffer lasts, no
+    allocation; `to_host()` reads the copies back afterwards as `fetch_device_result`-style dicts."""
+    FIELDS = {"key_off": np.int32, "key_valid": np.uint8, "agg_valid": np.uint8, "count": np.int64, "min": np.float64, "max": np.float64,
+              "avg": np.float64, "window_start_ms": np.int64, "window_end_ms": np.int64}
+
+    class _DeviceBytes:
+        def __init__(self, ptr, n):
+            self.__cuda_array_interface__ = {"shape": (n,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+
+    def __init__(self, torch, stream, device, reserve):
+        super().__init__()
+        self.torch, self.stream, self.device = torch, stream, device
+        self.buf, self.used = torch.empty(reserve, dtype=torch.uint8, device=device), 0
+
+    def take(self, w, r):
+        t = self.torch
+
+        def copy(ptr, n):
+            if self.used + n <= self.buf.numel():
+                dst = self.buf[self.used:self.used + n]
+                self.used += (n + 255) // 256 * 256
+            else:
+                dst = t.empty(n, dtype=t.uint8, device=self.device)
+            return dst.copy_(t.as_tensor(self._DeviceBytes(ptr, n), device=self.device), non_blocking=True) if n else dst
+        with t.cuda.stream(self.stream):
+            part = {f: copy(getattr(r, f), r.n_rows * np.dtype(dt).itemsize) for f, dt in self.FIELDS.items()}
+            part["key_bytes"] = copy(r.key_bytes, r.key_bytes_len)
+        self.append((r.key_bytes_len, part))
+
+    def to_host(self):
+        self.stream.synchronize()
+        out = []
+        for kb_len, part in self:
+            h = {f: part[f].cpu().numpy().view(dt) for f, dt in self.FIELDS.items()}
+            out.append({"key_off": np.append(h["key_off"], np.int32(kb_len)), "key_bytes": part["key_bytes"].cpu().numpy(),
+                        "key_valid": h["key_valid"], "agg_valid": h["agg_valid"], "count": h["count"], "min": h["min"], "max": h["max"],
+                        "avg": h["avg"], "window_start": h["window_start_ms"], "window_end": h["window_end_ms"]})
+        return out
+
+
+DUMP_ROWS = 1_000_000        # 7 float64 columns of this many rows: 56 MB per dump
+
+
+def dump_outputs(out_dir, parts, seed=0):
+    """Writes the rows of a step's device results (`fetch_device_result` dicts) as float64 arrays DIR/<column>.npy: window_start_ms,
+    window_end_ms, key_id, count, min, max, avg, sorted by (window start, key).  key_id is the key's rank among the distinct keys
+    of the step (-1 for a NULL key); min / max / avg are NaN where the aggregate is NULL.  Above DUMP_ROWS rows, a seeded sample
+    of row positions in that order is written, so two builds that emit the same rows write the same sample."""
+    import pyarrow as pa
+    import pyarrow.compute as pc
+    tabs = []
+    for p in parts:
+        n = len(p["count"])
+        if not n:
+            continue
+        keys = pa.Array.from_buffers(pa.binary(), n, [None, pa.py_buffer(p["key_off"]), pa.py_buffer(p["key_bytes"])])
+        keys = pc.if_else(pa.array(np.asarray(p["key_valid"]) != 0), keys, pa.scalar(None, pa.binary()))
+        null = np.asarray(p["agg_valid"]) == 0
+        tabs.append(pa.table({"window_start_ms": p["window_start"], "window_end_ms": p["window_end"], "key": keys, "count": p["count"],
+                              **{c: np.where(null, np.nan, np.asarray(p[c], np.float64)) for c in ("min", "max", "avg")}}))
+    cols = {"window_start_ms": pa.int64(), "window_end_ms": pa.int64(), "key": pa.binary(), "count": pa.int64(), "min": pa.float64(),
+            "max": pa.float64(), "avg": pa.float64()}
+    tab = pa.concat_tables(tabs) if tabs else pa.schema(cols).empty_table()
+    tab = tab.sort_by([("window_start_ms", "ascending"), ("key", "ascending")])
+    keys = pc.dictionary_encode(tab["key"].combine_chunks())
+    rank = np.full(len(keys.dictionary) + 1, -1.0)                  # the last entry stands for the NULL key
+    rank[pc.sort_indices(keys.dictionary).to_numpy()] = np.arange(len(keys.dictionary))
+    out = {c: tab[c].to_numpy().astype(np.float64) for c in cols if c != "key"}
+    out["key_id"] = rank[keys.indices.fill_null(len(keys.dictionary)).to_numpy()]
+    pick = np.arange(tab.num_rows)
+    if tab.num_rows > DUMP_ROWS:
+        pick = np.sort(np.random.default_rng(seed).choice(tab.num_rows, DUMP_ROWS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[pick])
+    return tab.num_rows, len(pick)
+
+
 def plan_e2e_steps(fit, warmup, steps, n_parity_ops):
     """How many warm-up and timed e2e steps run when `fit` operators (one per step, plus the parity pass) fit into device memory:
     at most 3 warm-ups and `steps` timed steps, never fewer than one of each."""
@@ -301,6 +384,9 @@ class Capture(list):
     def __init__(self, cut, window_ms):
         super().__init__()
         self.cut, self.window_ms = cut, window_ms
+
+    def take(self, w, r):
+        self.append(w.fetch_device_result(r, max_keys=0))
 
     def append(self, part):
         if isinstance(part, dict):
@@ -395,6 +481,8 @@ def main():
     if world != args.gpus:
         if world == 1 and args.gpus > 1:
             raise SystemExit("launch with torchrun --nproc-per-node N for --gpus N")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the output of one operator: run it with --gpus 1")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (no CPU fallback exists)")
     torch.cuda.set_device(local)
@@ -431,7 +519,7 @@ def main():
                     break
                 n_out += r.n_rows
                 if capture is not None:
-                    capture.append(w.fetch_device_result(r, max_keys=0))
+                    capture.take(w, r)
         # close the remaining windows a few at a time: one poll must stay below 2 GiB of key bytes (Utf8 offsets are 32-bit),
         # which 10 M 36-byte keys x 12 open sliding windows (cfg 5) would exceed
         step_ms = max(wl["slide_ms"] or wl["window_ms"], 1000) * (1 if G >= 4_000_000 else 64)
@@ -445,7 +533,7 @@ def main():
                     break
                 n_out += r.n_rows
                 if capture is not None:
-                    capture.append(w.fetch_device_result(r, max_keys=0))
+                    capture.take(w, r)
         return n_out
 
     def barrier():
@@ -465,14 +553,18 @@ def main():
     lazy = G >= 4_000_000
     wins = [None if lazy else new_window(d.capi.FLAG_KERNEL_TIMING) for _ in range(args.steps)]
     stats = []
+    dumped = None               # what the last timed step emits; room for ~4x the warm-up's rows (a poll re-reads its set's keys)
+    if args.dump_outputs:
+        room = 4 * out_rows * (len(StepCapture.FIELDS) * 8 + 40) + (64 << 20)
+        dumped = StepCapture(torch, stream, local, min(room, torch.cuda.mem_get_info()[0] // 4))
     sampler = ClockSampler(local); sampler.start()
     barrier()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(stream)
-    for w in wins:
+    for i, w in enumerate(wins):
         if lazy:
             w = new_window(d.capi.FLAG_KERNEL_TIMING)
-        step_device(w)
+        step_device(w, dumped if i == args.steps - 1 else None)
         if lazy:
             stats.append(w.stats()); w.close()
     ev1.record(stream)
@@ -484,6 +576,10 @@ def main():
         dist.all_gather_object(allms, round(ms / args.steps, 2))
         log(f"device-resident ms/step per rank: {allms}")
     log(f"device-resident: {ms / args.steps:.2f} ms/step")
+    if dumped is not None:
+        n_rows, n_dumped = dump_outputs(args.dump_outputs, dumped.to_host())
+        del dumped
+        log(f"last timed step: {n_rows} rows emitted, {n_dumped} written to {args.dump_outputs}")
     if not lazy:
         stats = [w.stats() for w in wins]
         for w in wins:

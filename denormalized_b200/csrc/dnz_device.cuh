@@ -79,6 +79,14 @@ constexpr unsigned long long ORD_F64_MAX = BITS_F64_MAX | SIGN64;        // ord(
 constexpr unsigned long long ORD_F64_MIN = ~(BITS_F64_MAX | SIGN64);     // ord(-MAX)
 __host__ __device__ __forceinline__ unsigned long long ord_bits(unsigned long long b) { return (b & SIGN64) ? ~b : (b | SIGN64); }
 __host__ __device__ __forceinline__ unsigned long long unord_bits(unsigned long long o) { return (o & SIGN64) ? (o & ~SIGN64) : ~o; }
+// The bits of a double through an opaque move.  Given __double_as_longlong(v), nvcc rewrites ord_bits' `b | SIGN64` into the
+// floating-point -|v| (DADD), which turns a NaN into the canonical 0x7FFFFFFFFFFFFFFF and so loses it from a totalOrder max.
+// Paths whose min / max see NaN take the bits from here.
+__device__ __forceinline__ unsigned long long f64_bits(double v) {
+  unsigned long long b;
+  asm("mov.b64 %0, %1;" : "=l"(b) : "d"(v));
+  return b;
+}
 // IEEE totalOrder key (arrow-ord cmp on floats == f64::total_cmp)
 __host__ __device__ __forceinline__ long long total_key(unsigned long long b) {
   long long s = (long long)b; return s ^ (long long)(((unsigned long long)(s >> 63)) >> 1);

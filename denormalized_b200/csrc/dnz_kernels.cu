@@ -648,7 +648,7 @@ cudaError_t launch_deferred(const AggParams& p, const DeferEntry* in, uint64_t n
 struct UAcc { double cnt, sum; unsigned long long mink, maxk, nulls; };
 __device__ __forceinline__ void uacc_add(UAcc& a, bool val_ok, double v) {
   if (!val_ok) { a.nulls++; return; }
-  const unsigned long long o = ord_bits((unsigned long long)__double_as_longlong(v));
+  const unsigned long long o = ord_bits(f64_bits(v));
   a.cnt += 1.0; a.sum += v; a.mink = max(a.mink, ~o); a.maxk = max(a.maxk, o);
 }
 __device__ void uacc_flush(UAcc& a, GroupState* m, GroupState* l, unsigned long long* nm, unsigned long long* nl, double* s_red) {
@@ -711,7 +711,7 @@ __global__ void __launch_bounds__(256) k_aggregate_ungrouped(const __grid_consta
         GroupState* d = k ? P.panes.late[pi] : P.panes.main[pi]; unsigned long long* dn = k ? P.panes.nullrows_late[pi] : P.panes.nullrows_main[pi];
         if (!d) continue;
         if (!val_ok) { if (dn) red_add_u64(dn, 1ull); continue; }
-        const unsigned long long o = ord_bits((unsigned long long)__double_as_longlong(v));
+        const unsigned long long o = ord_bits(f64_bits(v));
         red_add_f64(&d->cnt, 1.0); red_add_f64(&d->sum, v); red_max_u64(&d->minkey, ~o); red_max_u64(&d->maxkey, o);
       }
     }

@@ -43,3 +43,46 @@ def test_e2e_step_plan_fits_the_device():
         for par in (0, 1):
             w, s = b.plan_e2e_steps(fit, 5, 20, par)
             assert w >= 1 and s >= 1 and w + s + par <= max(fit, 2 + par)
+
+
+def test_dump_outputs_is_independent_of_emission_order(tmp_path):
+    """bench.py --dump-outputs: the same rows emitted in a different order and split into different polls write the same files,
+    sorted by (window start, key), with NULL keys and NULL aggregates kept apart; above DUMP_ROWS rows a fixed sample is written."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec); spec.loader.exec_module(b)
+    assert 7 * 8 * b.DUMP_ROWS <= 64 << 20
+    rng = np.random.default_rng(5)
+    rows = [(ws, key, int(rng.integers(1, 9)), float(rng.normal()), float(rng.normal()), float(rng.normal()))
+            for ws in (3000, 1000, 2000) for key in (b"sensor_9", b"sensor_10", None, b"k")]
+    rows[5] = rows[5][:2] + (0, None, None, None)
+
+    def parts(order, splits):
+        out = []
+        for chunk in np.array_split(np.array(order), splits):
+            rs = [rows[i] for i in chunk]
+            kb = b"pad" + b"".join(r[1] or b"" for r in rs)
+            off = np.cumsum([3] + [len(r[1] or b"") for r in rs]).astype(np.int32)
+            out.append({"key_off": off, "key_bytes": np.frombuffer(kb, np.uint8), "key_valid": np.array([r[1] is not None for r in rs], np.uint8),
+                        "count": np.array([r[2] for r in rs], np.int64), "min": np.array([r[3] or 0.0 for r in rs]),
+                        "max": np.array([r[4] or 0.0 for r in rs]), "avg": np.array([r[5] or 0.0 for r in rs]),
+                        "agg_valid": np.array([r[3] is not None for r in rs], np.uint8),
+                        "window_start": np.array([r[0] for r in rs], np.int64), "window_end": np.array([r[0] + 1000 for r in rs], np.int64)})
+        return out
+    n = len(rows)
+    assert b.dump_outputs(str(tmp_path / "a"), parts(range(n), 3)) == (n, n)
+    assert b.dump_outputs(str(tmp_path / "b"), parts(rng.permutation(n), 5)) == (n, n)
+    names = ["window_start_ms", "window_end_ms", "key_id", "count", "min", "max", "avg"]
+    got = {c: np.load(tmp_path / "a" / f"{c}.npy") for c in names}
+    for c in names:
+        assert got[c].dtype == np.float64 and np.array_equal(got[c], np.load(tmp_path / "b" / f"{c}.npy"), equal_nan=True), c
+    assert list(got["window_start_ms"]) == [1000.0] * 4 + [2000.0] * 4 + [3000.0] * 4
+    assert list(got["key_id"][:4]) == [0.0, 1.0, 2.0, -1.0]          # b"k" < b"sensor_10" < b"sensor_9", NULL last
+    null_row = (got["window_start_ms"] == 1000.0) & (got["key_id"] == 1.0)         # rows[5]: window 1000, b"sensor_10"
+    assert got["count"][null_row] == 0 and np.isnan(got["min"][null_row]).all()
+    b.DUMP_ROWS = 5
+    assert b.dump_outputs(str(tmp_path / "c"), parts(range(n), 2)) == (n, 5)
+    assert b.dump_outputs(str(tmp_path / "d"), parts(rng.permutation(n), 4)) == (n, 5)
+    for c in names:
+        assert np.array_equal(np.load(tmp_path / "c" / f"{c}.npy"), np.load(tmp_path / "d" / f"{c}.npy"), equal_nan=True), c
